@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...                          (the reference's CPU path, timed on host cores)
+    python bench.py ... --dump-outputs DIR                        (+ the last timed step's indices / scores as DIR/*.npy)
 
 A "step" = one batch of Q queries searched against the whole HBM-resident corpus (one pass of the hot path).
 Workload "headline" = BASELINE.json's metric shape: N=10M x d=1024 fp32, k=10, with configs[1]'s Q=64 cosine.
@@ -82,7 +83,13 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true", help="skip the untimed parity post-check")
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="N>1 candidate exchange: peer-memory kernels behind the C ABI (default) or NCCL all-gather + merge")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/indices.npy (row ids, float64) and DIR/scores.npy "
+                         "(float32), [Q x k]; inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU search's results: it needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -203,8 +210,7 @@ def cpu_reference_run(N_total, dim, dtype, Q, k, metric, budget_s=25.0, min_pass
     reference does not implement).  Threads pinned (OMP_PROC_BIND=close, set in main before libgomp starts); the
     median of >= 5 passes is reported.  Returns the JSON fields."""
     import numpy as np
-    import oracle
-    oracle.build()
+    import oracle  # loads the liboracle.so that build() made; never recompiles it (the tree may be read-only)
     hw = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
     # bounded sample: S rows of the same synthetic corpus (>= 1 GB of fp32 rows where the corpus is that large), Qs queries
     row_bytes = dim * 4
@@ -380,6 +386,7 @@ def measure(run: Runner, ix, n_shard, N_total, dim, dtype, Q, k, metric, steps, 
     t_wall0 = time.perf_counter()
     total_ms = run.timed_steps(lambda s: search_dev(q_all[warmup + s].data_ptr()), steps, flush)
     t_wall = time.perf_counter() - t_wall0
+    last = (out_idx.clone(), out_score.clone())  # the untimed searches below write into out_idx / out_score again
     scan_ms, scan_launches = ix.scan_time_ms()
     ix.enable_timing(False)
     launches = ix.stats()["kernel_launches"] - launches0 + (steps if G > 1 and not peer else 0)
@@ -405,7 +412,7 @@ def measure(run: Runner, ix, n_shard, N_total, dim, dtype, Q, k, metric, steps, 
            "scan_ms": scan_ms, "scan_launches": scan_launches, "launches": int(launches), "wall_s": t_wall, "clocks": clocks,
            "l2": "L2 flushed between steps (256 MB memset, untimed)" if flush is not None
                  else "corpus shard per GPU >> 126 MB L2 (inputs larger than L2; no flush needed)",
-           "out_idx": out_idx, "out_score": out_score, "q_all": q_all, "search_dev": search_dev}
+           "out_idx": out_idx, "out_score": out_score, "q_all": q_all, "search_dev": search_dev, "last": last}
 
     if want_e2e:
         # e2e: the reference-facing call with HOST buffers (H2D queries + D2H results inside the timed region)
@@ -426,17 +433,16 @@ def measure(run: Runner, ix, n_shard, N_total, dim, dtype, Q, k, metric, steps, 
             res_sc_h.copy_(out_score, non_blocking=True)
             torch.cuda.current_stream().synchronize()
 
-        e2e_steps = max(3, min(steps, 20))
         for i in range(min(warmup, 3)):
             step_e2e(i)
         t0 = time.perf_counter()
-        ev_ms = run.timed_steps(lambda s: step_e2e(warmup + (s % steps)), e2e_steps, None)
+        ev_ms = run.timed_steps(lambda s: step_e2e(warmup + s), steps, None)
         wall_ms = run.max_over_ranks((time.perf_counter() - t0) * 1e3)
         # G == 1: nk_search runs on the index's own stream and returns synchronously — the events on this stream see none
         # of it, the wall clock around the K calls is the honest figure.  G > 1: everything is ordered on the timed stream.
         e2e_ms = wall_ms if G == 1 else ev_ms
-        res["e2e"] = {"value": Q * e2e_steps / (e2e_ms / 1e3), "unit": "queries/s", "h2d_bytes_per_step": Q * dim * 4,
-                      "d2h_bytes_per_step": Q * k * 8, "ms_per_step": e2e_ms / e2e_steps, "steps": e2e_steps,
+        res["e2e"] = {"value": Q * steps / (e2e_ms / 1e3), "unit": "queries/s", "h2d_bytes_per_step": Q * dim * 4,
+                      "d2h_bytes_per_step": Q * k * 8, "ms_per_step": e2e_ms / steps, "steps": steps,
                       "timing": "wall clock around K synchronous nk_search calls (bracketed by barrier + synchronize)" if G == 1
                                 else "CUDA events on the launching stream around K steps (H2D, search, exchange, D2H, sync), MAX over ranks",
                       "api": "nk_search (C ABI, host buffers)" if G == 1 else
@@ -474,6 +480,23 @@ def roofline_of(res, n_shard, dim, dtype, Q, workload, peak, peak_src):
             r.update({"bound": "tensor", "achieved": tflops, "peak": tpeak, "unit": "TFLOP/s", "frac": tflops / tpeak, "peak_source": tsrc,
                       "hbm": {"achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak}})
     return r
+
+
+def dump_outputs(out_dir, out_idx, out_score, k_eff):
+    """--dump-outputs: the [Q x k'] result a caller of the device-resident search receives (k' = min(k, N)).  Row ids are
+    written as float64 (exact for 32-bit ids).  Results above 60 MB keep a fixed, seeded sample of the queries, whose
+    positions in the batch go to query_rows.npy."""
+    import numpy as np
+    idx = out_idx[:, :k_eff].cpu().numpy().view(np.uint32).astype(np.float64)
+    score = out_score[:, :k_eff].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    keep = (60 << 20) // (k_eff * 12 + 8)
+    if idx.shape[0] > keep:
+        rows = np.sort(np.random.default_rng(0).choice(idx.shape[0], keep, replace=False))
+        idx, score = idx[rows], score[rows]
+        np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "indices.npy"), idx)
+    np.save(os.path.join(out_dir, "scores.npy"), score)
 
 
 def also_entry(res, n, dim, dtype, Q, desc, peak, peak_src, workload):
@@ -699,6 +722,8 @@ def main():
         ix.fill_uniform(n_shard, CORPUS_SEED)
 
     res = measure(run, ix, n_shard, N_total, dim, dtype, Q, k, metric, args.steps, args.warmup, want_e2e=True, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *res["last"], min(k, N_total))
     used_path = res["path"]
     roofline = roofline_of(res, n_shard, dim, dtype, Q, args.workload, peak, peak_src)
     algo = roofline["algorithmic_bytes_per_launch"]
@@ -724,7 +749,7 @@ def main():
                                   "note": "asynchronous API: a first-stage overflow goes straight to the exact stage (exact_stage_rate); the TF32 retry stage belongs to the host-synchronous nk_search"}
     if not args.no_parity:
         line["parity_check"] = parity_check(run, ix, lo, hi, N_total, dim, dtype, Q, k, metric, res, clustered=clustered)
-    for key in ("out_idx", "out_score", "q_all", "search_dev"):
+    for key in ("out_idx", "out_score", "q_all", "search_dev", "last"):
         res.pop(key, None)
 
     # ---- the rest of the north_star grid (default N=1 line only), same timing rules, device-resident + e2e where cheap
@@ -737,7 +762,7 @@ def main():
                 index.set_path(path)
                 c0, s0 = index.debug_counters(), index.stats()["searches"]
                 r = measure(run, index, n, n, d, dt, q_, k_, m_, steps, warm, want_e2e=e2e)
-                for key in ("out_idx", "out_score", "q_all", "search_dev"):
+                for key in ("out_idx", "out_score", "q_all", "search_dev", "last"):
                     r.pop(key, None)
                 also[name] = also_entry(r, n, d, dt, q_, desc_, peak, peak_src, wl or name)
                 if r["path"] in ("shadow", "filter"):

@@ -81,3 +81,30 @@ def test_round2_bench_lines_carry_parity_check_and_grid():
     assert by["headline_8gpu_peer"]["exchange"].startswith("peer-memory")
     c5 = by["default_8gpu"]["also"]["c5"]  # configs[4] rides on the default 8-GPU command
     assert c5["parity_check"]["ok"] is True and c5["rows_per_gpu"] == 12_500_000 and c5["value"] > 0
+
+
+def test_dump_outputs_writes_the_result_as_npy(tmp_path):
+    import numpy as np
+    import torch
+    import bench
+    idx = torch.arange(12, dtype=torch.int32).reshape(3, 4)
+    idx[0, 0] = -1  # row id 2**32 - 1, as the C ABI's uint32 lands in the int32 buffer
+    score = torch.linspace(1, 0, 12).reshape(3, 4)
+    bench.dump_outputs(str(tmp_path / "a"), idx, score, 3)  # k' = min(k, N) = 3: the 4th column is never written
+    i, s = np.load(tmp_path / "a" / "indices.npy"), np.load(tmp_path / "a" / "scores.npy")
+    assert i.dtype == np.float64 and s.dtype == np.float32 and i.shape == s.shape == (3, 3)
+    assert i[0, 0] == 2 ** 32 - 1 and i[1].tolist() == [4, 5, 6] and (s == score[:, :3].numpy()).all()
+    assert not (tmp_path / "a" / "query_rows.npy").exists()
+    # above the size limit: the same seeded sample of queries every time, within 64 MB in all
+    Q, k = 600_000, 10
+    idx = torch.arange(Q * k, dtype=torch.int32).reshape(Q, k)
+    score = idx.float()
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), idx, score, k)
+    files = sorted(p.name for p in (tmp_path / "b").iterdir())
+    assert files == ["indices.npy", "query_rows.npy", "scores.npy"]
+    assert sum((tmp_path / "b" / f).stat().st_size for f in files) <= 64 << 20
+    rows = np.load(tmp_path / "b" / "query_rows.npy")
+    assert (np.diff(rows) > 0).all() and (rows == np.load(tmp_path / "c" / "query_rows.npy")).all()
+    i = np.load(tmp_path / "b" / "indices.npy")
+    assert (i == rows[:, None] * k + np.arange(k)).all()

@@ -55,3 +55,42 @@ def check_parity(rows, queries, k, metric, g_idx, g_score, o_idx, o_score, row_b
             f"exact scores of got {ex}, oracle {os_}")
         swaps += int((gi != oi).sum())
     return swaps
+
+
+def torch_fp64_topk(n, d, q, k, metric, slice_rows, rows_of_slice):
+    """Exact fp64 brute force at full size ON THE GPU (torch, fp64 matmul over row slices) — an arithmetic completely
+    independent of the kernels under test.  rows_of_slice(lo, cnt) -> float32 cuda tensor [cnt, d].  Returns (idx [Q, k]
+    int64 cpu, score [Q, k] float64 cpu) under the (score desc, row asc) / (distance asc, row asc) order."""
+    import torch
+    q64 = torch.from_numpy(np.asarray(q, dtype=np.float64)).cuda()
+    qn = q64.norm(dim=1)
+    best_s = best_i = None
+    for lo in range(0, n, slice_rows):
+        cnt = min(slice_rows, n - lo)
+        x = rows_of_slice(lo, cnt).double()
+        s = x @ q64.T  # [cnt, Q]
+        if metric == "cosine":
+            den = x.norm(dim=1)[:, None] * qn[None, :]
+            s = torch.where(den > 0, s / den, torch.zeros_like(s))
+        elif metric == "euclidean":
+            s = -((x * x).sum(1)[:, None] + (q64 * q64).sum(1)[None, :] - 2.0 * s)
+        kk = min(k + 8, cnt)
+        v, i = torch.topk(s, kk, dim=0)  # [kk, Q]
+        i = i + lo
+        if best_s is None:
+            best_s, best_i = v, i
+        else:
+            best_s, best_i = torch.cat([best_s, v]), torch.cat([best_i, i])
+            keep = torch.topk(best_s, min(k + 8, best_s.shape[0]), dim=0).indices
+            best_s, best_i = torch.gather(best_s, 0, keep), torch.gather(best_i, 0, keep)
+        del x, s
+    # final order: score desc, row asc
+    bs, bi = best_s.T.cpu().numpy(), best_i.T.cpu().numpy()
+    out_i = np.empty((bs.shape[0], k), dtype=np.int64)
+    out_s = np.empty((bs.shape[0], k), dtype=np.float64)
+    for r in range(bs.shape[0]):
+        order = np.lexsort((bi[r], -bs[r]))[:k]
+        out_i[r], out_s[r] = bi[r][order], bs[r][order]
+    if metric == "euclidean":
+        out_s = np.sqrt(np.maximum(-out_s, 0.0))
+    return out_i, out_s

@@ -6,18 +6,18 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-BIN = os.path.join(ROOT, "tests", "cpp", "host_mirror_test")
 
 
 @pytest.fixture(scope="module")
-def host_binary(knn_lib):
+def host_binary(knn_lib, tmp_path_factory):
+    # Built fresh into a temporary directory: the source tree may be read-only, and a binary left there from an earlier
+    # build could be linked against another copy of the library.
     src = os.path.join(ROOT, "tests", "cpp", "host_mirror_test.cpp")
-    hdr = os.path.join(ROOT, "nornicdb_b200", "host", "nornic_cuda.hpp")
     lib = os.path.join(ROOT, "nornicdb_b200", "libnornic_knn.so")
-    if not os.path.exists(BIN) or any(os.path.getmtime(f) > os.path.getmtime(BIN) for f in (src, hdr, lib)):
-        subprocess.run(["/usr/bin/g++", "-std=c++17", "-O1", "-Wall", "-I", ROOT, src, "-L", os.path.dirname(lib), "-lnornic_knn",
-                        f"-Wl,-rpath,{os.path.dirname(lib)}", "-lpthread", "-o", BIN], check=True, cwd=ROOT)
-    return BIN
+    out = str(tmp_path_factory.mktemp("host_mirror") / "host_mirror_test")
+    subprocess.run(["/usr/bin/g++", "-std=c++17", "-O1", "-Wall", "-I", ROOT, src, "-L", os.path.dirname(lib), "-lnornic_knn",
+                    f"-Wl,-rpath,{os.path.dirname(lib)}", "-lpthread", "-o", out], check=True, cwd=ROOT)
+    return out
 
 
 def test_host_mirror_error_paths_without_gpu(host_binary):

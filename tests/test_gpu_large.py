@@ -5,7 +5,7 @@ independent kernels (CUDA-core, 3xTF32 tensor, 1xTF32-filter + rescoring), and i
 import numpy as np
 import pytest
 
-from parity import check_parity, exact_scores_for
+from parity import check_parity, exact_scores_for, torch_fp64_topk
 
 pytestmark = pytest.mark.gpu
 
@@ -146,45 +146,6 @@ def test_config4_fp16_l2_full_size(knn_lib, oracle_mod):
     assert np.allclose(gs[0], want_dist, rtol=1e-4)
 
 
-def _torch_fp64_topk(n, d, q, k, metric, slice_rows, rows_of_slice):
-    """Exact fp64 brute force at full size ON THE GPU (torch, fp64 matmul over row slices) — an arithmetic completely
-    independent of the kernels under test.  rows_of_slice(lo, cnt) -> float32 cuda tensor [cnt, d].  Returns (idx [Q, k]
-    int64 cpu, score [Q, k] float64 cpu) under the (score desc, row asc) / (distance asc, row asc) order."""
-    import torch
-    q64 = torch.from_numpy(np.asarray(q, dtype=np.float64)).cuda()
-    qn = q64.norm(dim=1)
-    best_s = best_i = None
-    for lo in range(0, n, slice_rows):
-        cnt = min(slice_rows, n - lo)
-        x = rows_of_slice(lo, cnt).double()
-        s = x @ q64.T  # [cnt, Q]
-        if metric == "cosine":
-            den = x.norm(dim=1)[:, None] * qn[None, :]
-            s = torch.where(den > 0, s / den, torch.zeros_like(s))
-        elif metric == "euclidean":
-            s = -((x * x).sum(1)[:, None] + (q64 * q64).sum(1)[None, :] - 2.0 * s)
-        kk = min(k + 8, cnt)
-        v, i = torch.topk(s, kk, dim=0)  # [kk, Q]
-        i = i + lo
-        if best_s is None:
-            best_s, best_i = v, i
-        else:
-            best_s, best_i = torch.cat([best_s, v]), torch.cat([best_i, i])
-            keep = torch.topk(best_s, min(k + 8, best_s.shape[0]), dim=0).indices
-            best_s, best_i = torch.gather(best_s, 0, keep), torch.gather(best_i, 0, keep)
-        del x, s
-    # final order: score desc, row asc
-    bs, bi = best_s.T.cpu().numpy(), best_i.T.cpu().numpy()
-    out_i = np.empty((bs.shape[0], k), dtype=np.int64)
-    out_s = np.empty((bs.shape[0], k), dtype=np.float64)
-    for r in range(bs.shape[0]):
-        order = np.lexsort((bi[r], -bs[r]))[:k]
-        out_i[r], out_s[r] = bi[r][order], bs[r][order]
-    if metric == "euclidean":
-        out_s = np.sqrt(np.maximum(-out_s, 0.0))
-    return out_i, out_s
-
-
 def test_config3_full_size_all_queries_fp64(knn_lib, oracle_mod):
     """BASELINE.json configs[2] at FULL size: N=10M d=1024 fp32, ALL 1024 queries, k=100, inner product (the CTA-pair
     path), against an fp64 brute force over all 10^7 x 1024 (row, query) pairs computed slice by slice with torch on the
@@ -204,7 +165,7 @@ def test_config3_full_size_all_queries_fp64(knn_lib, oracle_mod):
         torch.cuda.synchronize()
         return x
 
-    oi, os_ = _torch_fp64_topk(n, d, q, k, "dot", 500_000, rows_of_slice)
+    oi, os_ = torch_fp64_topk(n, d, q, k, "dot", 500_000, rows_of_slice)
     swaps = check_parity(lambda idx: np.stack([ix.read_rows(int(r), 1)[0] for r in idx]), q, k, "dot", gi, gs, oi, os_)
     ix.release()
     assert swaps <= 8, swaps  # boundary swaps (fp64 scores closer than fp32 summation noise) are counted, not hidden
@@ -231,7 +192,7 @@ def test_clustered_corpus_1m_rows_fp64(knn_lib, oracle_mod):
         assert ix.debug_flags()[0] == 0
     counters = ix.debug_counters()
     ix.release()
-    oi, os_ = _torch_fp64_topk(n, d, q, k, "cosine", 250_000, lambda lo, cnt: torch.from_numpy(host[lo:lo + cnt]).cuda())
+    oi, os_ = torch_fp64_topk(n, d, q, k, "cosine", 250_000, lambda lo, cnt: torch.from_numpy(host[lo:lo + cnt]).cuda())
     for path, (gi, gs) in res.items():
         check_parity(host, q, k, "cosine", gi, gs, oi, os_, swap_eps=5e-6)
     assert (res["shadow"][0] == res["filter"][0]).all()

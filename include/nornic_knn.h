@@ -248,6 +248,29 @@ int nk_merge_keys_device(int device_id, const uint64_t *keys_dev, uint32_t n_lis
 int nk_index_set_row_groups(NkIndex *ix, const uint32_t *group_of_row, uint64_t n_rows, uint32_t n_groups);
 int nk_search_groups(NkIndex *ix, const float *query_host, uint32_t k, uint32_t *out_group, uint32_t *out_row, float *out_score);
 
+/* Cluster-routed search (ClusterIndex.SearchWithClusters, pkg/gpu/kmeans.go:816-836), single-device indexes.
+ * nk_index_set_clusters installs a clustering: K <= NK_MAX_CLUSTERS centroids [K x dim] fp32 (host) and one assignment per row
+ * (host int32 [n_rows], n_rows == rows of the index); entries outside [0, K) put the row in no cluster; centroids == NULL
+ * clears.  The device keeps the centroids and the members sorted by (cluster, row) (built on the device, rows are read in
+ * place).  Cleared by every row-count changing mutation (upload / append / remove_swap / fill / attach), like the row groups;
+ * update_row keeps it (the new contents are scored, the assignment is the caller's business).
+ * nk_search_clusters answers Q queries at once.  Per query: route to the P = min(n_probe, K) centroids nearest in squared
+ * Euclidean distance (float32 differences, float64 squares), nearest first, ties to the lower centroid id (FindNearestClusters,
+ * kmeans.go:734-777); score exactly in fp32, with the index's metric, every member of those clusters that the row mask admits,
+ * score floor honoured; return the best k, ordered by (score desc | distance asc), ties by position in the candidate list
+ * (probe rank, then ascending row: the order GetClusterMembers + SearchCandidates see).  out_idx / out_score [Q x k]; slots
+ * beyond a query's candidate count hold 0xffffffff / 0.  out_probe (nullable) [Q x P] = the routed clusters.  Returns
+ * min(k, rows of the index) (0 for k == 0, Q == 0 or an empty index) or -1: k > NK_MAX_K, n_probe == 0, several devices,
+ * "no clusters set".  Host-synchronous (one synchronisation).  The _device form is asynchronous on `stream` (NULL = the
+ * index's own), with device pointers, no host round trip and no allocation per call; overflow of an internal capacity is
+ * reported by nk_index_status. */
+#define NK_MAX_CLUSTERS 4096u
+int nk_index_set_clusters(NkIndex *ix, const float *centroids_host, uint32_t K, const int32_t *assign_host, uint64_t n_rows);
+int nk_search_clusters(NkIndex *ix, const float *queries_host, uint32_t Q, uint32_t k, uint32_t n_probe, uint32_t *out_idx,
+                       float *out_score, int32_t *out_probe);
+int nk_search_clusters_device(NkIndex *ix, const float *queries_dev, uint32_t Q, uint32_t k, uint32_t n_probe, uint32_t *out_idx_dev,
+                              float *out_score_dev, int32_t *out_probe_dev, void *stream);
+
 /* Row-sharded search, one rank per GPU, exchange BEHIND the ABI (SURVEY.md §8e; the reference has a single DeviceID,
  * gpu.go:218).  Each rank owns rows [row_base, row_base + n) (nk_index_set_row_base).  The only data that crosses GPUs is
  * every rank's Q*k candidate keys, pushed with plain peer stores over NVLink into a small buffer each rank exports through

@@ -91,6 +91,9 @@ SIGNATURES = {
     "nk_index_status": (_i, [_vp, _vp]),
     "nk_index_set_row_groups": (_i, [_vp, _vp, _u64, C.c_uint32]),
     "nk_search_groups": (_i, [_vp, _vp, C.c_uint32, _vp, _vp, _vp]),
+    "nk_index_set_clusters": (_i, [_vp, _vp, C.c_uint32, _vp, _u64]),
+    "nk_search_clusters": (_i, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp]),
+    "nk_search_clusters_device": (_i, [_vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _vp, _vp, _vp, _vp]),
     "nk_comm_create": (_vp, [_i, _i, _i, _sz]),
     "nk_comm_export": (_i, [_vp, _vp]),
     "nk_comm_connect": (_i, [_vp, _vp]),

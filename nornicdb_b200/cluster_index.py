@@ -5,7 +5,9 @@ algorithm run on the GPU against the HBM-resident corpus, nothing is copied back
   * assignment  = `nk_index_assign_nearest`: the fused scan with the roles swapped (centroids are the indexed corpus,
     the corpus rows are the queries, k = 1)                                   — kmeans.go:458-546
   * update      = `nk_index_cluster_means`: float64 per-cluster sums on device  — kmeans.go:585-618
-  * cluster-restricted search = `nk_score_subset` over the members            — kmeans.go:816-895
+  * cluster-restricted search = `nk_search_clusters`: routing, member gather and the exact scan of the probed clusters'
+    rows in one device call for a whole batch (the clustering is installed lazily, `nk_index_set_clusters`)
+                                                                              — kmeans.go:816-895
 Centroid bookkeeping (K x dim, tiny) stays on the host in the reference's arithmetic (float32 differences, float64
 squares: squaredEuclidean kmeans.go:430-454).
 
@@ -25,6 +27,7 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 
 from .embedding_index import EmbeddingIndex, ErrInvalidDimensions, SearchResult
+from .knn import NK_MAX_K
 
 
 class ErrInvalidK(ValueError):  # kmeans.go ErrInvalidK
@@ -93,6 +96,7 @@ class ClusterIndex(EmbeddingIndex):
         self.iterations = 0
         self.clusterIterations = 0
         self.centroidDrift = 0.0
+        self._dev_stale = True  # the device's copy of (centroids, assignments) must be re-installed before a routed search
 
     # ---- initialisation (kmeans.go:335-427) ------------------------------------------------------------------------
     def _init_rows(self, n: int) -> np.ndarray:
@@ -151,6 +155,7 @@ class ClusterIndex(EmbeddingIndex):
                 if changed == 0:
                     break
             self.centroids, self.assignments = cen, assign
+            self._dev_stale = True
             self._build_cluster_map()
             self.clustered = True
             self.lastClusterTime = time.time()
@@ -174,6 +179,7 @@ class ClusterIndex(EmbeddingIndex):
             self.pendingUpdates = []
             self.clustered = False
             self.updatesSinceCluster = 0
+            self._dev_stale = True
 
     def IsClustered(self) -> bool:
         return self.clustered
@@ -214,13 +220,67 @@ class ClusterIndex(EmbeddingIndex):
     def SearchWithClusters(self, query, topK: int, numClusters: int) -> Optional[List[SearchResult]]:  # kmeans.go:816-836
         if not self.IsClustered():
             return self.Search(query, topK)
-        ids = self.FindNearestClusters(query, numClusters)
+        q = np.asarray(query, dtype=np.float32).reshape(-1)
+        if q.size != self.dimensions:
+            raise ErrInvalidDimensions()
+        return self.SearchWithClustersBatch(q.reshape(1, -1), topK, numClusters)[0]
+
+    def SearchWithClustersBatch(self, queries, topK: int, numClusters: int) -> List[Optional[List[SearchResult]]]:
+        """SearchWithClusters for every row of `queries` [Q x dim], one device call for the whole batch."""
+        q = np.ascontiguousarray(np.asarray(queries, dtype=np.float32))
+        if q.ndim != 2 or q.shape[1] != self.dimensions:
+            raise ErrInvalidDimensions()
+        if not self.IsClustered():
+            return [self.Search(v, topK) for v in q]
+        with self.mu:
+            topK, numClusters = int(topK), int(numClusters)
+            # the two cases the device call cannot serve: k above NK_MAX_K, and an assignment array that no longer covers
+            # exactly the index's rows (Add without OnNodeUpdate, Remove: the reference leaves those inconsistent too).
+            # KnnIndex always has search_clusters; an index stand-in that only scores subsets (the CPU test double of the
+            # host-logic tests) is served by the same subset path the reference takes.
+            if (numClusters <= 0 or topK <= 0 or topK > NK_MAX_K or len(self.assignments) != len(self._ix)
+                    or not hasattr(self._ix, "search_clusters")):
+                return [self._search_with_clusters_host(v, topK, numClusters) for v in q]
+            if self._dev_stale:
+                self._ix.set_clusters(self.centroids, self.assignments)
+                self._dev_stale = False
+            idx, sc = self._ix.search_clusters(q, topK, numClusters)
+            out: List[Optional[List[SearchResult]]] = []
+            for i in range(q.shape[0]):
+                hit = idx[i] != 0xFFFFFFFF  # slots beyond the candidate count (topK clamped to it, kmeans.go:852-855)
+                out.append([SearchResult(self.nodeIDs[int(r)], float(s), float(1.0 - s)) for r, s in zip(idx[i][hit], sc[i][hit])]
+                           if hit.any() else None)
+            return out
+
+    def _search_with_clusters_host(self, q: np.ndarray, topK: int, numClusters: int) -> Optional[List[SearchResult]]:
+        ids = self.FindNearestClusters(q, numClusters)
         if not ids:
             return None
         cand = self.GetClusterMembers(ids)
         if not cand:
             return None
-        return self.SearchCandidates(query, cand, topK)
+        return self.SearchCandidates(q, cand, topK)
+
+    # Row-count changing mutations clear the device's clustering: re-install it before the next routed search.
+    def Add(self, nodeID: str, embedding) -> None:
+        with self.mu:
+            self._dev_stale = True
+            super().Add(nodeID, embedding)
+
+    def AddBatch(self, nodeIDs: Sequence[str], embeddings) -> None:
+        with self.mu:
+            self._dev_stale = True
+            super().AddBatch(nodeIDs, embeddings)
+
+    def Remove(self, nodeID: str) -> bool:
+        with self.mu:
+            self._dev_stale = True
+            return super().Remove(nodeID)
+
+    def Deserialize(self, data: bytes) -> None:
+        with self.mu:
+            self._dev_stale = True
+            super().Deserialize(data)
 
     def SearchCandidates(self, query, candidateIndices: Sequence[int], topK: int) -> Optional[List[SearchResult]]:  # kmeans.go:839-895
         q = np.asarray(query, dtype=np.float32).reshape(-1)
@@ -257,6 +317,7 @@ class ClusterIndex(EmbeddingIndex):
                 self.assignments = np.append(self.assignments, np.int32(new))
                 self.clusterMap.setdefault(new, []).append(idx)
             self.updatesSinceCluster += 1
+            self._dev_stale = True
 
     def ShouldRecluster(self) -> bool:  # kmeans.go:980-1005
         if not self.clustered:
@@ -277,6 +338,7 @@ class ClusterIndex(EmbeddingIndex):
             for c in affected:
                 if counts[c] > 0:
                     self.centroids[c] = fresh[c]
+            self._dev_stale = True
 
     def Dimensions(self) -> int:
         return self.dimensions

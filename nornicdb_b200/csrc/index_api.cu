@@ -53,6 +53,8 @@ struct NkShard {
     uint32_t *group = nullptr;  // node id per row (nk_index_set_row_groups), local rows
     size_t group_bytes = 0;
     bool group_on = false;
+    nk::ClusterLayout clusters;  // nk_index_set_clusters (single-device indexes)
+    nk::ClusterSearchWs cws;
     nk::Workspace ws;
     uint64_t *h_keys = nullptr;  // pinned staging for multi-shard host merge
     size_t h_keys_bytes = 0;
@@ -100,11 +102,11 @@ struct NkIndex {
     }
 };
 
-// Row-count changing mutations invalidate the row mask (its bits are positions).
+// Row-count changing mutations invalidate the row mask (its bits are positions), the row groups and the clustering.
 static void drop_row_mask(NkIndex *ix) {
     ix->mask_on = false;
     ix->n_groups = 0;
-    for (auto &s : ix->shards) { s.mask_on = false; s.group_on = false; }
+    for (auto &s : ix->shards) { s.mask_on = false; s.group_on = false; s.clusters.on = false; }
 }
 
 static void shard_drop_shadow(NkShard &s) {
@@ -459,6 +461,8 @@ void nk_index_release(NkIndex *ix) {
         if (s.cvt) cudaFree(s.cvt);
         if (s.mask) cudaFree(s.mask);
         if (s.group) cudaFree(s.group);
+        s.clusters.release();
+        s.cws.release();
         s.ws.release();
     }
     delete ix;
@@ -1338,6 +1342,117 @@ int nk_search_groups(NkIndex *ix, const float *query_host, uint32_t k, uint32_t 
     uint32_t found = 0;
     while (found < ke && out_group[found] != 0xffffffffu) ++found;
     return (int)found;
+}
+
+// ---- cluster-routed search (ClusterIndex.SearchWithClusters, kmeans.go:816-836; cluster_search.cu) ---------------------------
+int nk_index_set_clusters(NkIndex *ix, const float *centroids_host, uint32_t K, const int32_t *assign_host, uint64_t n_rows) {
+    nk::DeviceGuard _restore_device;
+    NkShard *s;
+    if (single_shard(ix, &s)) return -1;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    if (!centroids_host) {
+        s->clusters.on = false;
+        return 0;
+    }
+    if (K == 0 || K > NK_MAX_CLUSTERS) { nk::set_error("nk_index_set_clusters: K=%u outside [1, NK_MAX_CLUSTERS=%u]", K, NK_MAX_CLUSTERS); return -1; }
+    if (n_rows != s->n) { nk::set_error("nk_index_set_clusters: %llu assignments, index has %llu rows", (unsigned long long)n_rows, (unsigned long long)s->n); return -1; }
+    if (n_rows && !assign_host) { nk::set_error("null argument"); return -1; }
+    NK_CUDA_OK(cudaSetDevice(s->device));
+    if (nk::cluster_layout_build(s->clusters, centroids_host, K, ix->dim, assign_host, n_rows, s->stream, &ix->stats.kernel_launches)) return -1;
+    ix->stats.bytes_h2d += (uint64_t)K * ix->dim * 4 + n_rows * 4;
+    return 0;
+}
+
+static int search_clusters_impl(NkIndex *ix, NkShard *s, const float *q_dev, uint32_t Q, uint32_t k, uint32_t n_probe, uint32_t *out_idx_dev,
+                                float *out_score_dev, int32_t *out_probe_dev, cudaStream_t st) {
+    nk::ClusterSearchArgs a;
+    a.rows = s->rows; a.dtype = ix->dtype; a.dim = ix->dim; a.row_base = s->base;
+    a.row_mask = s->mask_on ? s->mask : nullptr; a.min_score = ix->key_floor(); a.metric = ix->metric;
+    a.queries = q_dev; a.Q = Q; a.k = k; a.n_probe = n_probe;
+    a.out_idx = out_idx_dev; a.out_score = out_score_dev; a.out_probe = out_probe_dev;
+    a.flags = s->ws.flags; a.stream = st;
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev;
+    a.timing = ix->timing_on; a.timing_events = &ev;
+    NK_RANGE_PUSH("nk_search_clusters");
+    const int rc = nk::cluster_search(s->di, s->clusters, a, s->cws, &ix->stats.kernel_launches);
+    NK_RANGE_POP();
+    for (auto &e : ev) {
+        s->timing.push_back(e);
+        s->timing_launches.push_back(1);
+    }
+    ix->last_path = NK_PATH_SIMT;
+    ix->stats.searches++;
+    ix->stats.queries += Q;
+    return rc;
+}
+
+// Shared argument checks; returns 1 when there is nothing to search (k == 0, Q == 0 or no rows), 0 to go on, -1 on error.
+static int clusters_precheck(NkIndex *ix, NkShard *s, uint32_t Q, uint32_t k, uint32_t n_probe) {
+    if (k > NK_MAX_K) { nk::set_error("nk_search_clusters: k=%u exceeds NK_MAX_K=%u", k, NK_MAX_K); return -1; }
+    if (n_probe == 0) { nk::set_error("nk_search_clusters: n_probe must be >= 1"); return -1; }
+    if (k == 0 || Q == 0 || s->n == 0) return 1;
+    if (!s->clusters.on) { nk::set_error("nk_search_clusters: no clusters set (nk_index_set_clusters)"); return -1; }
+    (void)ix;
+    return 0;
+}
+
+int nk_search_clusters(NkIndex *ix, const float *queries_host, uint32_t Q, uint32_t k, uint32_t n_probe, uint32_t *out_idx, float *out_score,
+                       int32_t *out_probe) {
+    nk::DeviceGuard _restore_device;
+    NkShard *s;
+    if (single_shard(ix, &s)) return -1;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    const int pre = clusters_precheck(ix, s, Q, k, n_probe);
+    if (pre) return pre < 0 ? -1 : 0;
+    if (!queries_host || !out_idx || !out_score) { nk::set_error("null argument"); return -1; }
+    NK_CUDA_OK(cudaSetDevice(s->device));
+    const uint32_t P = std::min(n_probe, s->clusters.K);
+    const size_t qbytes = (size_t)Q * ix->dim * 4, rbytes = (size_t)Q * k * 4, pbytes = (size_t)Q * P * 4;
+    if (nk::ws_reserve((void **)&s->ws.queries, &s->ws.queries_bytes, qbytes)) return -1;
+    if (nk::ws_reserve((void **)&s->ws.out_idx, &s->ws.out_idx_bytes, rbytes + pbytes)) return -1;
+    if (nk::ws_reserve((void **)&s->ws.out_score, &s->ws.out_score_bytes, rbytes)) return -1;
+    int32_t *d_probe = reinterpret_cast<int32_t *>(s->ws.out_idx + (size_t)Q * k);
+    const size_t need = 2 * rbytes + pbytes + sizeof(int) * nk::NK_FLAG_WORDS;
+    if (s->h_res_bytes < need) {
+        if (s->h_res) cudaFreeHost(s->h_res);
+        s->h_res = nullptr; s->h_res_bytes = 0;
+        NK_CUDA_OK(cudaMallocHost((void **)&s->h_res, need + need / 4));
+        s->h_res_bytes = need + need / 4;
+    }
+    NK_CUDA_OK(cudaMemcpyAsync(s->ws.queries, queries_host, qbytes, cudaMemcpyHostToDevice, s->stream));
+    ix->stats.bytes_h2d += qbytes;
+    if (search_clusters_impl(ix, s, s->ws.queries, Q, k, n_probe, s->ws.out_idx, s->ws.out_score, d_probe, s->stream)) return -1;
+    // results, probe lists and status words come back through one pinned buffer and ONE synchronisation
+    int *hflags = reinterpret_cast<int *>(s->h_res + 2 * rbytes + pbytes);
+    NK_CUDA_OK(cudaMemcpyAsync(s->h_res, s->ws.out_idx, rbytes + pbytes, cudaMemcpyDeviceToHost, s->stream));
+    NK_CUDA_OK(cudaMemcpyAsync(s->h_res + rbytes + pbytes, s->ws.out_score, rbytes, cudaMemcpyDeviceToHost, s->stream));
+    NK_CUDA_OK(cudaMemcpyAsync(hflags, s->ws.flags, sizeof(int) * nk::NK_FLAG_WORDS, cudaMemcpyDeviceToHost, s->stream));
+    NK_CUDA_OK(cudaStreamSynchronize(s->stream));
+    ix->stats.bytes_d2h += 2 * rbytes + pbytes;
+    if (hflags[nk::FLAG_FATAL]) {
+        cudaMemsetAsync(s->ws.flags, 0, sizeof(int), s->stream);
+        nk::set_error("internal: candidate buffer overflow (flag=%d)", hflags[nk::FLAG_FATAL]);
+        return -1;
+    }
+    memcpy(out_idx, s->h_res, rbytes);
+    if (out_probe) memcpy(out_probe, s->h_res + rbytes, pbytes);
+    memcpy(out_score, s->h_res + rbytes + pbytes, rbytes);
+    return (int)std::min<uint64_t>(k, s->n);
+}
+
+int nk_search_clusters_device(NkIndex *ix, const float *queries_dev, uint32_t Q, uint32_t k, uint32_t n_probe, uint32_t *out_idx_dev,
+                              float *out_score_dev, int32_t *out_probe_dev, void *stream) {
+    nk::DeviceGuard _restore_device;
+    NkShard *s;
+    if (single_shard(ix, &s)) return -1;
+    std::lock_guard<std::mutex> lk(ix->mu);
+    const int pre = clusters_precheck(ix, s, Q, k, n_probe);
+    if (pre) return pre < 0 ? -1 : 0;
+    if (!queries_dev || !out_idx_dev || !out_score_dev) { nk::set_error("null argument"); return -1; }
+    NK_CUDA_OK(cudaSetDevice(s->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (search_clusters_impl(ix, s, queries_dev, Q, k, n_probe, out_idx_dev, out_score_dev, out_probe_dev, st)) return -1;
+    return (int)std::min<uint64_t>(k, s->n);
 }
 
 // ---- row-sharded search with the exchange behind the ABI (exchange.cu) ----------------------------------------------------

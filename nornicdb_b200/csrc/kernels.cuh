@@ -1,5 +1,8 @@
 // kernels.cuh — internal launcher interface between the C-ABI host code and the kernels.
 #pragma once
+#include <utility>
+#include <vector>
+
 #include "common.cuh"
 
 namespace nk {
@@ -87,10 +90,11 @@ int scan_simt(const DeviceInfo &di, const ScanArgs &a, Workspace &ws, uint64_t *
 // key(list l, query q, slot i) = keys[l*list_stride + q*q_stride + i], i < list_len (0 = k).
 // only_if != nullptr: the kernel returns at once unless *only_if != 0 (device-side conditional fallback).
 // dec_idx / dec_score != nullptr: also write the decoded (index, score) arrays [Q x k] (fused decode_keys; dec_metric).
+// q_lists != nullptr (device [Q]): query q merges only its first q_lists[q] <= n_lists lists.
 int merge_keys(const uint64_t *keys, uint32_t n_lists, size_t list_stride, size_t q_stride, uint32_t Q, uint32_t k,
                uint64_t *out_keys, cudaStream_t stream, const int *only_if = nullptr, uint32_t list_len = 0,
                uint32_t *dec_idx = nullptr, float *dec_score = nullptr, int dec_metric = 0, const uint32_t *wait_flags = nullptr,
-               uint32_t wait_epoch = 0, int *wait_err = nullptr);
+               uint32_t wait_epoch = 0, int *wait_err = nullptr, const uint32_t *q_lists = nullptr);
 // keys [Q][k] -> idx/score [Q][k]; euclidean decodes score = sqrt(-s).
 int decode_keys(const uint64_t *keys, uint32_t Q, uint32_t k, int metric, uint32_t *out_idx, float *out_score,
                 cudaStream_t stream, const int *only_if = nullptr);
@@ -124,5 +128,49 @@ int count_changed(const int32_t *a, const uint32_t *b, uint64_t n, unsigned long
 int convert_f32_to_16(const float *src, void *dst, int dtype, size_t n, cudaStream_t s);  // fp16 / bf16, round to nearest even like the host's astype
 int gather_rows(const void *rows, int dtype, uint32_t dim, const uint32_t *idx, uint32_t n_idx, void *out,
                 cudaStream_t s);
+
+// ---- cluster-routed search (cluster_search.cu) ----------------------------------------------------------------------------
+// Device layout of an installed clustering: centroids [K x dim], CSR offsets [K+1] and member rows (local ids) sorted by
+// (cluster, row).  Rows assigned outside [0, K) belong to no cluster.  Host copies of the sizes the planner needs.
+struct ClusterLayout {
+    float *centroids = nullptr;   size_t centroids_bytes = 0;
+    uint32_t *offs = nullptr;     size_t offs_bytes = 0;
+    uint32_t *members = nullptr;  size_t members_bytes = 0;
+    void *build = nullptr;        size_t build_bytes = 0;  // counting-sort scratch (per-tile histograms, assignments)
+    uint32_t K = 0, max_rows = 0;
+    uint64_t n_assigned = 0;
+    bool on = false;
+    void release();
+};
+int cluster_layout_build(ClusterLayout &L, const float *centroids_host, uint32_t K, uint32_t dim, const int32_t *assign_host,
+                         uint64_t n_rows, cudaStream_t s, uint64_t *launches);
+
+// Grow-only scratch of the routed search: one arena carved per call, plus the route kernel's per-query-group arrival
+// counters (zero between calls: the last CTA of a group resets its own).
+struct ClusterSearchWs {
+    void *arena = nullptr;      size_t arena_bytes = 0;
+    int *counters = nullptr;    size_t counters_bytes = 0;
+    uint64_t *cand = nullptr;   size_t cand_bytes = 0;
+    int release();
+};
+struct ClusterSearchArgs {
+    const void *rows = nullptr;
+    int dtype = NK_DTYPE_F32;
+    uint32_t dim = 0;
+    uint64_t row_base = 0;
+    const uint32_t *row_mask = nullptr;
+    float min_score = -INFINITY;  // key space
+    int metric = NK_METRIC_COSINE;
+    const float *queries = nullptr;  // device [Q x dim]
+    uint32_t Q = 0, k = 0, n_probe = 0;
+    uint32_t *out_idx = nullptr;  // device [Q x k]
+    float *out_score = nullptr;
+    int32_t *out_probe = nullptr;  // device [Q x min(n_probe, K)] or nullptr
+    int *flags = nullptr;
+    cudaStream_t stream = nullptr;
+    bool timing = false;  // record an event pair around every scan launch into *timing_events
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> *timing_events = nullptr;
+};
+int cluster_search(const DeviceInfo &di, const ClusterLayout &L, const ClusterSearchArgs &a, ClusterSearchWs &ws, uint64_t *launches);
 
 }  // namespace nk

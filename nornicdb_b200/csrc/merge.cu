@@ -27,6 +27,7 @@ struct MergeParams {
     const uint32_t *wait_flags;
     uint32_t wait_epoch;
     int *wait_err;  // set to 2 if a peer did not arrive within ~2 s (never spin forever: a hung GPU is a strike)
+    const uint32_t *q_lists;  // optional: query q merges only its first q_lists[q] lists (cluster-routed search)
 };
 
 // One CTA per query.  Streams the n_lists*k candidate keys through a 2048-wide sort buffer, keeping
@@ -39,7 +40,7 @@ __global__ void __launch_bounds__(MERGE_THREADS) merge_keys_kernel(MergeParams p
     __shared__ int s_fill;
     const uint32_t q = blockIdx.x;
     const uint64_t *base = p.keys + (size_t)q * p.q_stride;
-    const uint64_t total = (uint64_t)p.n_lists * p.list_len;
+    const uint64_t total = (uint64_t)(p.q_lists ? p.q_lists[q] : p.n_lists) * p.list_len;
     const int tid = threadIdx.x;
     if (p.wait_flags) {
         // fused exchange wait: thread l polls peer l's arrival word (system-scope acquire), bounded by a wall-clock timeout
@@ -238,7 +239,7 @@ __global__ void __launch_bounds__(MERGE_THREADS) merge_keys_kernel(MergeParams p
 
 int merge_keys(const uint64_t *keys, uint32_t n_lists, size_t list_stride, size_t q_stride, uint32_t Q, uint32_t k,
                uint64_t *out_keys, cudaStream_t stream, const int *only_if, uint32_t list_len, uint32_t *dec_idx, float *dec_score,
-               int dec_metric, const uint32_t *wait_flags, uint32_t wait_epoch, int *wait_err) {
+               int dec_metric, const uint32_t *wait_flags, uint32_t wait_epoch, int *wait_err, const uint32_t *q_lists) {
     if (Q == 0 || k == 0) return 0;
     if (k > MERGE_P / 2) {
         set_error("merge: k=%u too large", k);
@@ -249,7 +250,7 @@ int merge_keys(const uint64_t *keys, uint32_t n_lists, size_t list_stride, size_
         return -1;
     }
     MergeParams p{keys, n_lists, list_stride, q_stride, k, out_keys, only_if, list_len ? list_len : k, dec_idx, dec_score, dec_metric,
-                  wait_flags, wait_epoch, wait_err};
+                  wait_flags, wait_epoch, wait_err, q_lists};
     NK_CUDA_OK(launch_pdl(merge_keys_kernel, dim3(Q), dim3(MERGE_THREADS), 0, stream, true, p));
     return 0;
 }

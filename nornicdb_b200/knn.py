@@ -16,6 +16,7 @@ METRICS = {"cosine": 0, "dot": 1, "euclidean": 2}
 DTYPES = {"f32": 0, "fp32": 0, "float32": 0, "f16": 1, "fp16": 1, "float16": 1, "bf16": 2, "bfloat16": 2}
 PATHS = {"auto": 0, "simt": 1, "tensor": 2, "filter": 3, "shadow": 4}
 NK_MAX_K = 1024
+NK_MAX_CLUSTERS = 4096
 
 
 class KnnError(RuntimeError):
@@ -37,6 +38,7 @@ class KnnIndex:
         # bf16 rows travel as raw uint16 bit patterns (numpy has no bfloat16): see to_bf16_bits / from_bf16_bits
         self.np_dtype = np.float16 if self.dtype == 1 else np.uint16 if self.dtype == 2 else np.float32
         self.devices = list(devices)
+        self._clusters_k = 0  # K of the last clustering installed (nk_index_set_clusters)
         ids = (C.c_int * len(self.devices))(*self.devices)
         self.ptr = self.lib.nk_index_create(ids, len(self.devices), self.dim, self.dtype, METRICS[metric])
         if not self.ptr:
@@ -245,6 +247,48 @@ class KnnIndex:
                                              len(r), kk, idx.ctypes.data_as(C.c_void_p),
                                              sc.ctypes.data_as(C.c_void_p)), "nk_score_subset")
         return idx[:ke], sc[:ke]
+
+    # ---- cluster-routed search (ClusterIndex.SearchWithClusters, kmeans.go:816-836) -------------------------------
+    def set_clusters(self, centroids, assign) -> None:
+        """Install a clustering for search_clusters: centroids [K x dim] and one int32 assignment per row (values outside
+        [0, K) belong to no cluster).  None clears.  Row-count changing mutations clear it; update_row keeps it."""
+        if centroids is None:
+            _check(self.lib.nk_index_set_clusters(self.ptr, None, 0, None, 0), "nk_index_set_clusters")
+            self._clusters_k = 0
+            return
+        c = np.ascontiguousarray(np.asarray(centroids, dtype=np.float32))
+        if c.ndim != 2 or c.shape[1] != self.dim:
+            raise KnnError(f"invalid dimensions: centroids {c.shape}, index has {self.dim}")
+        a = np.ascontiguousarray(np.asarray(assign, dtype=np.int32).reshape(-1))
+        _check(self.lib.nk_index_set_clusters(self.ptr, c.ctypes.data_as(C.c_void_p), c.shape[0], a.ctypes.data_as(C.c_void_p), a.size),
+               "nk_index_set_clusters")
+        self._clusters_k = c.shape[0]
+
+    def search_clusters(self, queries, k: int, n_probe: int, return_probes: bool = False):
+        """Route each query to its n_probe nearest centroids and search their members exactly.  Returns (idx [Q x k'],
+        score [Q x k']) with k' = min(k, rows), and the probe lists [Q x min(n_probe, K)] when return_probes."""
+        q = np.ascontiguousarray(np.asarray(queries, dtype=np.float32))
+        if q.ndim == 1:
+            q = q.reshape(1, -1)
+        if q.shape[1] != self.dim:
+            raise KnnError(f"invalid dimensions: query has {q.shape[1]}, index has {self.dim}")
+        Q, k, n_probe = q.shape[0], int(k), int(n_probe)
+        idx = np.empty((Q, max(k, 0)), dtype=np.uint32)
+        sc = np.empty((Q, max(k, 0)), dtype=np.float32)
+        probes = np.empty((Q, max(n_probe, 0)), dtype=np.int32)
+        ke = _check(self.lib.nk_search_clusters(self.ptr, q.ctypes.data_as(C.c_void_p), Q, max(k, 0), max(n_probe, 0),
+                                                idx.ctypes.data_as(C.c_void_p), sc.ctypes.data_as(C.c_void_p),
+                                                probes.ctypes.data_as(C.c_void_p)), "nk_search_clusters")
+        if not return_probes:
+            return idx[:, :ke], sc[:, :ke]
+        P = min(n_probe, self._clusters_k) if ke else 0  # the probe lists are packed with row stride P
+        return idx[:, :ke], sc[:, :ke], probes.reshape(-1)[:Q * P].reshape(Q, P)
+
+    def search_clusters_device(self, q_ptr: int, Q: int, k: int, n_probe: int, out_idx_ptr: int, out_score_ptr: int,
+                               out_probe_ptr: int = 0, stream: int = 0) -> int:
+        """Device-resident, asynchronous on `stream`: out arrays [Q x k] (and [Q x min(n_probe, K)] probes, optional)."""
+        return _check(self.lib.nk_search_clusters_device(self.ptr, q_ptr, Q, k, n_probe, out_idx_ptr, out_score_ptr, out_probe_ptr or None,
+                                                         stream), "nk_search_clusters_device")
 
     # ---- k-means routing on device (pkg/gpu/kmeans.go) ----------------------------------------------------------
     def assign_nearest(self, centroids, assign: np.ndarray, metric: str = "euclidean") -> int:

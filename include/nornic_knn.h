@@ -310,6 +310,19 @@ int nk_score_subset(NkIndex *ix, const float *query_host, const uint32_t *rows_h
 int nk_index_assign_nearest(NkIndex *ix, const float *centroids_host, uint32_t K, int metric, int32_t *assign_io,
                             uint64_t *changed);
 int nk_index_cluster_means(NkIndex *ix, const int32_t *assign_host, uint32_t K, float *centroids_io, uint32_t *counts_out);
+/* k-means++ seeding (initCentroidsKMeansPlusPlus, kmeans.go:364-427) over every row of an fp32 index, on the device.
+ * Centroid 0 = row first_row.  For c = 1 .. K-1: D2[i] = min over chosen centroids of squaredEuclidean(row i, centroid)
+ * (float32 differences, float64 squares); target = draws[c-1] * sum(D2) in float64; centroid c = the first row i with
+ * cumsum(D2)[0..i] >= target, or the last row when there is none (NaN total).  A row whose distance to the new centroid
+ * is not strictly smaller keeps its D2 (strict <, kmeans.go:414-421).  draws (host, [K-1], values in [0, 1)) are the
+ * caller's uniform variates (rand.Float64), so the result is reproducible.  centroids_out (host, [K x dim]) = those
+ * rows; rows_out (nullable, [K]) = their row positions in the index (first_row's numbering, across all shards);
+ * rows_scored (nullable) = how many (row, step) distances were computed rather than skipped by the triangle-inequality
+ * bound.  Every row takes part, and the row mask is not consulted (like nk_index_assign_nearest).  Multi-device indexes
+ * are supported.  Returns 0, or -1 for: a non-fp32 index, K == 0, K > rows, first_row >= rows, or draws == NULL with
+ * K > 1. */
+int nk_index_kmeanspp(NkIndex *ix, uint32_t K, uint64_t first_row, const double *draws, float *centroids_out,
+                      uint32_t *rows_out, uint64_t *rows_scored);
 
 /* Synthetic fp32 query block from the shared generator, on the device of a single-device index. */
 int nk_fill_uniform_device(int device_id, float *out_dev, uint64_t n_rows, uint32_t dim, uint64_t seed,

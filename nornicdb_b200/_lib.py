@@ -81,6 +81,7 @@ SIGNATURES = {
     "nk_blob_vectors": (_i, [_vp, C.c_size_t, _vp, _vp, _vp]),
     "nk_index_assign_nearest": (_i, [_vp, _vp, C.c_uint32, _i, _vp, _vp]),
     "nk_index_cluster_means": (_i, [_vp, _vp, C.c_uint32, _vp, _vp]),
+    "nk_index_kmeanspp": (_i, [_vp, C.c_uint32, _u64, _vp, _vp, _vp, _vp]),
     "nk_fill_uniform_device": (_i, [_i, _vp, _u64, C.c_uint32, _u64, _u64, _vp]),
     "nk_index_fill_clustered": (_i, [_vp, _u64, _u64, C.c_uint32, C.c_float, _i]),
     "nk_index_refresh_shadow": (_i, [_vp]),

@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libnornic_knn.so")
-SOURCES = ["runtime.cu", "rowops.cu", "merge.cu", "scan_simt.cu", "scan_tensor.cu", "scan_tensor_shadow.cu", "scan_tensor_pair.cu", "assign_tensor.cu", "cluster_search.cu", "exchange.cu", "legacy_abi.cu", "index_api.cu"]
+SOURCES = ["runtime.cu", "rowops.cu", "merge.cu", "scan_simt.cu", "scan_tensor.cu", "scan_tensor_shadow.cu", "scan_tensor_pair.cu", "assign_tensor.cu", "cluster_search.cu", "kmeanspp.cu", "exchange.cu", "legacy_abi.cu", "index_api.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

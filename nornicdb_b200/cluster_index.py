@@ -8,12 +8,15 @@ algorithm run on the GPU against the HBM-resident corpus, nothing is copied back
   * cluster-restricted search = `nk_search_clusters`: routing, member gather and the exact scan of the probed clusters'
     rows in one device call for a whole batch (the clustering is installed lazily, `nk_index_set_clusters`)
                                                                               — kmeans.go:816-895
+  * k-means++ seeding = `nk_index_kmeanspp`: D² weighting over every row, one streaming pass per centroid that skips
+    rows the triangle inequality rules out                                    — kmeans.go:364-427
 Centroid bookkeeping (K x dim, tiny) stays on the host in the reference's arithmetic (float32 differences, float64
 squares: squaredEuclidean kmeans.go:430-454).
 
 Deviations, stated: the reference seeds k-means++ / random init from Go's global math/rand stream, which cannot be
-reproduced; this mirror takes a numpy Generator (seedable) and, for corpora above `init_sample` rows, runs k-means++ on
-a uniform sample of the rows read back from the device.  `assign` selects which of the reference's two assignment rules
+reproduced; this mirror takes a numpy Generator (seedable): k-means++ draws the first row and then one uniform variate
+per centroid from it.  Only index stand-ins without `kmeanspp` seed on the host (`_init_kmeanspp`), and above
+`init_sample` rows they do so on a uniform sample of the rows read back.  `assign` selects which of the reference's two assignment rules
 is used: "euclidean" (assignToCentroids, the CPU definition) or "cosine" (assignToCentroidsGPU, what the reference runs
 when its GPU manager is enabled).
 """
@@ -142,6 +145,10 @@ class ClusterIndex(EmbeddingIndex):
                 cen = np.array(initial_centroids, dtype=np.float32, order="C", copy=True)
                 if cen.shape != (k, self.dimensions):
                     raise ValueError(f"initial_centroids must be [{k} x {self.dimensions}]")
+            elif self.config.InitMethod == "kmeans++" and hasattr(self._ix, "kmeanspp"):
+                # every row takes part (kmeans.go:364-427); the same draws, in the same order, as _init_kmeanspp takes
+                first = int(self.rng.integers(n))
+                cen, _, _ = self._ix.kmeanspp(k, first, self.rng.random(k - 1))
             else:
                 rows = self._init_rows(n)
                 cen = self._init_kmeanspp(k, rows) if self.config.InitMethod == "kmeans++" else self._init_random(k, rows)

@@ -1274,6 +1274,187 @@ int nk_index_cluster_means(NkIndex *ix, const int32_t *assign_host, uint32_t K, 
     return 0;
 }
 
+// ---- k-means++ seeding on device (initCentroidsKMeansPlusPlus, kmeans.go:364-427; kmeanspp.cu, DESIGN.md §3.8) ---------
+// Each shard carves its grow-only scratch into d2 / near / block sums / centroids / cc / draws / picks.  A single-device
+// index queues all K - 1 steps on one stream and synchronises once.  A multi-device index picks the shard of each
+// selection on the host from the shard totals, summed in shard order; shards are contiguous row ranges, so the global
+// cumulative order is the single-device one.  That costs one synchronisation per step.
+namespace {
+struct KppShard {
+    NkShard *s = nullptr;
+    uint64_t first = 0;  // index position of the shard's row 0
+    double *d2 = nullptr, *bsum = nullptr, *cc = nullptr, *draws = nullptr, *total = nullptr;
+    int32_t *near = nullptr;
+    float *cen = nullptr;
+    uint32_t *sel = nullptr;
+    unsigned long long *scored = nullptr;
+    long long *pick = nullptr;
+};
+}  // namespace
+
+static int kmeanspp_steps(NkIndex *ix, std::vector<KppShard> &kv, uint32_t K, uint64_t first_row, const double *draws,
+                          float *centroids_out, uint32_t *rows_out, uint64_t *rows_scored) {
+    const uint32_t dim = ix->dim;
+    const size_t row_bytes = (size_t)dim * 4;
+    auto update = [&](KppShard &k, uint32_t c, bool init) {
+        ix->stats.kernel_launches++;
+        return nk::kpp_update(k.s->di, static_cast<const float *>(k.s->rows), k.s->n, dim, k.cen, c, init, k.cc, k.d2, k.near,
+                              k.bsum, k.scored, k.s->stream);
+    };
+    auto cc = [&](KppShard &k, uint32_t c) {
+        ix->stats.kernel_launches++;
+        return nk::kpp_cc(k.cen, c, dim, k.cc, k.s->stream);
+    };
+    std::vector<uint64_t> picked(K, first_row);
+    if (kv.size() == 1) {  // every step queued back to back on one stream
+        KppShard &k = kv[0];
+        NkShard &s = *k.s;
+        const float *rows = static_cast<const float *>(s.rows);
+        NK_CUDA_OK(cudaSetDevice(s.device));
+        if (K > 1) NK_CUDA_OK(cudaMemcpyAsync(k.draws, draws, (size_t)(K - 1) * 8, cudaMemcpyHostToDevice, s.stream));
+        NK_CUDA_OK(cudaMemcpyAsync(k.cen, rows + (first_row - k.first) * dim, row_bytes, cudaMemcpyDeviceToDevice, s.stream));
+        if (K > 1 && update(k, 0, true)) return -1;
+        for (uint32_t c = 1; c < K; ++c) {
+            ix->stats.kernel_launches++;
+            if (nk::kpp_select(nk::KPP_SELECT, k.d2, k.bsum, s.n, k.draws, c, 0.0, 0.0, rows, dim, k.cen, k.sel, nullptr, nullptr, s.stream))
+                return -1;
+            if (c + 1 < K && (cc(k, c) || update(k, c, false))) return -1;  // no update after the last selection
+        }
+        std::vector<uint32_t> sel(K);
+        NK_CUDA_OK(cudaMemcpyAsync(centroids_out, k.cen, (size_t)K * row_bytes, cudaMemcpyDeviceToHost, s.stream));
+        NK_CUDA_OK(cudaMemcpyAsync(sel.data(), k.sel, (size_t)K * 4, cudaMemcpyDeviceToHost, s.stream));
+        NK_CUDA_OK(cudaStreamSynchronize(s.stream));
+        for (uint32_t c = 1; c < K; ++c) picked[c] = k.first + sel[c];
+    } else {
+        // the chosen row travels through the host to every shard's centroid array
+        std::vector<float> crow(dim);
+        std::vector<double> tot(kv.size());
+        auto fetch_row = [&](KppShard &k, uint64_t local) -> int {
+            NK_CUDA_OK(cudaSetDevice(k.s->device));
+            NK_CUDA_OK(cudaMemcpy(crow.data(), static_cast<const float *>(k.s->rows) + local * dim, row_bytes, cudaMemcpyDeviceToHost));
+            return 0;
+        };
+        auto place = [&](uint32_t c) -> int {
+            for (auto &k : kv) {
+                NK_CUDA_OK(cudaSetDevice(k.s->device));
+                NK_CUDA_OK(cudaMemcpyAsync(k.cen + (size_t)c * dim, crow.data(), row_bytes, cudaMemcpyHostToDevice, k.s->stream));
+                if (c + 1 < K && ((c > 0 && cc(k, c)) || update(k, c, c == 0))) return -1;
+            }
+            return 0;
+        };
+        for (auto &k : kv)
+            if (first_row >= k.first && first_row < k.first + k.s->n && fetch_row(k, first_row - k.first)) return -1;
+        if (place(0)) return -1;
+        for (uint32_t c = 1; c < K; ++c) {
+            for (size_t j = 0; j < kv.size(); ++j) {
+                KppShard &k = kv[j];
+                NK_CUDA_OK(cudaSetDevice(k.s->device));
+                ix->stats.kernel_launches++;
+                if (nk::kpp_select(nk::KPP_TOTAL, k.d2, k.bsum, k.s->n, nullptr, c, 0.0, 0.0, nullptr, dim, nullptr, nullptr, k.total,
+                                   nullptr, k.s->stream))
+                    return -1;
+                NK_CUDA_OK(cudaMemcpyAsync(&tot[j], k.total, 8, cudaMemcpyDeviceToHost, k.s->stream));
+            }
+            double total = 0.0;
+            for (size_t j = 0; j < kv.size(); ++j) {
+                NK_CUDA_OK(cudaSetDevice(kv[j].s->device));
+                NK_CUDA_OK(cudaStreamSynchronize(kv[j].s->stream));
+                total += tot[j];
+            }
+            const double target = draws[c - 1] * total;
+            // the first shard whose offset + total reaches the target selects at that offset; one whose in-shard scan
+            // falls short by rounding passes on to the next; none (NaN total) -> the last row
+            long long pick = -1;
+            size_t js = kv.size() - 1;
+            double off = 0.0;
+            for (size_t j = 0; j < kv.size() && pick < 0; ++j) {
+                KppShard &k = kv[j];
+                if (off + tot[j] >= target) {
+                    NK_CUDA_OK(cudaSetDevice(k.s->device));
+                    ix->stats.kernel_launches++;
+                    if (nk::kpp_select(nk::KPP_SELECT_AT, k.d2, k.bsum, k.s->n, nullptr, c, target, off, nullptr, dim, nullptr, nullptr,
+                                       nullptr, k.pick, k.s->stream))
+                        return -1;
+                    NK_CUDA_OK(cudaMemcpyAsync(&pick, k.pick, 8, cudaMemcpyDeviceToHost, k.s->stream));
+                    NK_CUDA_OK(cudaStreamSynchronize(k.s->stream));
+                    if (pick >= 0) js = j;
+                }
+                off += tot[j];
+            }
+            const uint64_t local = pick >= 0 ? (uint64_t)pick : kv[js].s->n - 1;
+            picked[c] = kv[js].first + local;
+            if (fetch_row(kv[js], local) || place(c)) return -1;
+        }
+        NK_CUDA_OK(cudaSetDevice(kv[0].s->device));
+        NK_CUDA_OK(cudaMemcpyAsync(centroids_out, kv[0].cen, (size_t)K * row_bytes, cudaMemcpyDeviceToHost, kv[0].s->stream));
+        NK_CUDA_OK(cudaStreamSynchronize(kv[0].s->stream));
+    }
+    uint64_t scored = 0;
+    for (auto &k : kv) {
+        unsigned long long v = 0;
+        NK_CUDA_OK(cudaSetDevice(k.s->device));
+        NK_CUDA_OK(cudaMemcpyAsync(&v, k.scored, 8, cudaMemcpyDeviceToHost, k.s->stream));
+        NK_CUDA_OK(cudaStreamSynchronize(k.s->stream));
+        scored += v;
+    }
+    if (rows_scored) *rows_scored = scored;
+    if (rows_out)
+        for (uint32_t c = 0; c < K; ++c) rows_out[c] = (uint32_t)picked[c];
+    ix->stats.bytes_d2h += (uint64_t)K * row_bytes;
+    return 0;
+}
+
+int nk_index_kmeanspp(NkIndex *ix, uint32_t K, uint64_t first_row, const double *draws, float *centroids_out, uint32_t *rows_out,
+                      uint64_t *rows_scored) {
+    nk::DeviceGuard _restore_device;
+    if (!ix || !centroids_out) { nk::set_error("null argument"); return -1; }
+    if (ix->dtype != NK_DTYPE_F32) { nk::set_error("nk_index_kmeanspp: fp32 index required"); return -1; }
+    if (K == 0) { nk::set_error("nk_index_kmeanspp: K must be >= 1"); return -1; }
+    std::lock_guard<std::mutex> lk(ix->mu);
+    const uint64_t N = ix->rows();
+    if (K > N) { nk::set_error("nk_index_kmeanspp: K=%u exceeds the %llu rows", K, (unsigned long long)N); return -1; }
+    if (first_row >= N) { nk::set_error("nk_index_kmeanspp: first_row %llu out of range", (unsigned long long)first_row); return -1; }
+    if (K > 1 && !draws) { nk::set_error("nk_index_kmeanspp: K > 1 needs draws"); return -1; }
+    NK_RANGE_PUSH("nk_index_kmeanspp");
+    struct Pop { ~Pop() { NK_RANGE_POP(); } } pop_on_exit;
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    std::vector<KppShard> kv;
+    uint64_t pos = 0;
+    for (auto &s : ix->shards) {
+        if (s.n == 0) continue;
+        NK_CUDA_OK(cudaSetDevice(s.device));
+        const uint64_t nblk = (s.n + nk::KPP_BLOCK - 1) / nk::KPP_BLOCK;
+        const size_t kd = (size_t)K * ix->dim * 4;
+        if (nk::ws_reserve(&s.ws.scratch, &s.ws.scratch_bytes, al(s.n * 8) + al(s.n * 4) + al(nblk * 8) + al(kd) + 2 * al((size_t)K * 8) +
+                                                                   al((size_t)K * 4) + 256))
+            return -1;
+        unsigned char *p = static_cast<unsigned char *>(s.ws.scratch);
+        KppShard k;
+        k.s = &s;
+        k.first = pos;
+        k.d2 = reinterpret_cast<double *>(p);          p += al(s.n * 8);
+        k.near = reinterpret_cast<int32_t *>(p);       p += al(s.n * 4);
+        k.bsum = reinterpret_cast<double *>(p);        p += al(nblk * 8);
+        k.cen = reinterpret_cast<float *>(p);          p += al(kd);
+        k.cc = reinterpret_cast<double *>(p);          p += al((size_t)K * 8);
+        k.draws = reinterpret_cast<double *>(p);       p += al((size_t)K * 8);
+        k.sel = reinterpret_cast<uint32_t *>(p);       p += al((size_t)K * 4);
+        k.scored = reinterpret_cast<unsigned long long *>(p);
+        k.total = reinterpret_cast<double *>(p + 8);
+        k.pick = reinterpret_cast<long long *>(p + 16);
+        NK_CUDA_OK(cudaMemsetAsync(k.scored, 0, 8, s.stream));
+        kv.push_back(k);
+        pos += s.n;
+    }
+    const int rc = kmeanspp_steps(ix, kv, K, first_row, draws, centroids_out, rows_out, rows_scored);
+    for (auto &k : kv) {  // nothing stays queued on an error path
+        cudaSetDevice(k.s->device);
+        cudaStreamSynchronize(k.s->stream);
+    }
+    if (rc != 0) cudaGetLastError();
+    return rc;
+}
+
 // ---- best-of-chunks per node (db.index.vector.queryNodes, call_vector.go:177-256; SURVEY.md §8(f)2) -------------------------
 // Rows are chunk embeddings; group_of_row[r] = the node row r belongs to (ids in [0, n_groups)).  Stays set until a
 // row-count changing mutation (like the row mask, whose bits are positions).

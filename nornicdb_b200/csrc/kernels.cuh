@@ -125,6 +125,24 @@ int decode_group_keys(const uint64_t *keys, uint32_t k, int metric, const uint32
 int cluster_sums(const float *rows, uint64_t n, uint32_t dim, const int32_t *assign, uint32_t K, double *sums,
                  unsigned long long *counts, cudaStream_t s);
 int count_changed(const int32_t *a, const uint32_t *b, uint64_t n, unsigned long long *changed, cudaStream_t s);
+
+// ---- k-means++ seeding (kmeanspp.cu) --------------------------------------------------------------------------------------
+// Per shard: d2 [n] fp64 (distance to the nearest chosen centroid), near [n] (its index), bsum [ceil(n / KPP_BLOCK)] fp64
+// block sums of d2, cen [K x dim] the chosen centroids, cc [K] fp64 distances from the newest centroid to the earlier ones.
+constexpr uint32_t KPP_BLOCK = 1024;  // rows per fixed partial-sum block
+// d2 <- min(d2, squaredEuclidean(row, cen[c])) (strict <), skipping rows the triangle-inequality bound rules out; init:
+// d2 <- squaredEuclidean(row, cen[0]) for every row.  Rewrites bsum; *scored += rows whose distance was computed.
+int kpp_update(const DeviceInfo &di, const float *rows, uint64_t n, uint32_t dim, const float *cen, uint32_t c, bool init,
+               const double *cc, double *d2, int32_t *near, double *bsum, unsigned long long *scored, cudaStream_t s);
+// Selection of centroid c, one CTA.  mode KPP_SELECT: target = draws[c-1] * total, copies the chosen row into cen[c] and
+// its local id into sel[c] (n - 1 when no row reaches the target).  KPP_TOTAL: *total_out = sum of bsum.  KPP_SELECT_AT:
+// the given target and offset of this shard, *pick_out = the chosen local row or -1 when none reaches the target.
+enum { KPP_SELECT = 0, KPP_TOTAL = 1, KPP_SELECT_AT = 2 };
+int kpp_select(int mode, const double *d2, const double *bsum, uint64_t n, const double *draws, uint32_t c, double target,
+               double offset, const float *rows, uint32_t dim, float *cen, uint32_t *sel, double *total_out, long long *pick_out,
+               cudaStream_t s);
+// cc[j] = sqrt(squaredEuclidean(cen[c], cen[j])) for j < c.
+int kpp_cc(const float *cen, uint32_t c, uint32_t dim, double *cc, cudaStream_t s);
 int convert_f32_to_16(const float *src, void *dst, int dtype, size_t n, cudaStream_t s);  // fp16 / bf16, round to nearest even like the host's astype
 int gather_rows(const void *rows, int dtype, uint32_t dim, const uint32_t *idx, uint32_t n_idx, void *out,
                 cudaStream_t s);

@@ -315,6 +315,22 @@ class KnnIndex:
                                                counts.ctypes.data_as(C.c_void_p)), "nk_index_cluster_means")
         return c, counts
 
+    def kmeanspp(self, K: int, first_row: int, draws) -> Tuple[np.ndarray, np.ndarray, int]:
+        """initCentroidsKMeansPlusPlus over every row, on the device: centroid 0 is row `first_row`, centroid c is chosen
+        by the uniform variate draws[c-1] in [0, 1).  Returns (centroids float32 [K x dim], their rows uint32 [K], how
+        many (row, step) distances were computed rather than skipped)."""
+        K = int(K)
+        d = np.ascontiguousarray(np.asarray(draws, dtype=np.float64).reshape(-1))
+        if K >= 1 and d.size != K - 1:
+            raise KnnError(f"kmeanspp: {d.size} draws for K={K} (need K - 1)")
+        cen = np.empty((max(K, 0), self.dim), dtype=np.float32)
+        rows = np.empty(max(K, 0), dtype=np.uint32)
+        scored = C.c_uint64(0)
+        _check(self.lib.nk_index_kmeanspp(self.ptr, max(K, 0), int(first_row), d.ctypes.data_as(C.c_void_p) if d.size else None,
+                                          cen.ctypes.data_as(C.c_void_p), rows.ctypes.data_as(C.c_void_p), C.byref(scored)),
+               "nk_index_kmeanspp")
+        return cen, rows, int(scored.value)
+
 
 def to_bf16_bits(a) -> np.ndarray:
     """fp32 array -> bf16 bit patterns (uint16), round to nearest even (what the device conversion does)."""
